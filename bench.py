@@ -17,6 +17,8 @@ The same line carries, under "configs", the other BASELINE.json configurations m
                           1 sample per GPU at N = 8 as BASELINE names it)
   cc12m_256x256_ddim50    configs[4]: DDIM 50-step sampling, batch 16 per GPU, no collective
 Prints ONE JSON line. `--only <name>` / `--config/--batch` restrict the run (development aid).
+`--dump-outputs DIR` writes what the headline's last timed step computed as DIR/<name>.npy (see dump_outputs), so
+that two builds can be compared output for output: weights, inputs and random draws depend only on the arguments.
 """
 import argparse
 import gc
@@ -195,8 +197,61 @@ def timed(ctx, fn, steps):
     return e0.elapsed_time(e1)
 
 
-def measure_train(ctx, cfg_name, B, steps, warmup, headline=False, mixed_ratio=None):
-    """fwd+bwd sample-steps/s of one configuration at ctx.world GPUs; B = per-GPU batch."""
+DUMP_IMAGE_ELEMS = 1 << 21  # larger image-shaped outputs are dumped at this many fixed positions
+DUMP_GRAD_ELEMS = 4096      # gradient elements dumped per parameter
+DUMP_MAX_BYTES = 64 << 20
+
+
+def _fixed_positions(t, n, seed):
+    """`t` flattened, at `n` positions drawn from a fixed seed (all of it when it has no more than `n` elements)."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= n:
+        return flat
+    g = torch.Generator().manual_seed(seed)
+    idx = torch.randint(flat.numel(), (n,), generator=g).sort().values
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(path, outputs, vm):
+    """Writes what one training step returned to its caller: get_loss's (loss, time, x_t, prediction, target[,
+    weights]) and the parameter gradients. Image-shaped arrays above DUMP_IMAGE_ELEMS elements are written as
+    <name>_sample.npy at fixed positions; gradients as grad_norms.npy (float64, one per parameter) and
+    grad_sample.npy (DUMP_GRAD_ELEMS fixed positions of each parameter, zero-padded), in the order of
+    grad_names.txt. The gradients are read from the engine's gradient arena, which holds the last backward's
+    result until the next backward starts."""
+    import numpy as np
+
+    from mdm_b200.models import native
+
+    names = ["loss", "time", "x_t", "pred", "target", "weights"]
+    arrays = {}
+    for i, (name, t) in enumerate(zip(names, outputs)):
+        if t is None:
+            continue
+        dt = torch.float64 if t.dtype in (torch.int64, torch.float64) else torch.float32
+        if t.numel() > DUMP_IMAGE_ELEMS:
+            name, t = name + "_sample", _fixed_positions(t, DUMP_IMAGE_ELEMS, i)
+        arrays[name] = t.detach().to(dt).cpu().numpy()
+    nn_ = vm.native()
+    grads = native.arena_views(nn_.active_arena, nn_.params, nn_.offsets)
+    arrays["grad_norms"] = torch.stack([g.double().norm() for g in grads]).cpu().numpy()
+    sample = torch.zeros(len(grads), DUMP_GRAD_ELEMS, device=grads[0].device)
+    for i, g in enumerate(grads):
+        s = _fixed_positions(g, DUMP_GRAD_ELEMS, i)
+        sample[i, :s.numel()] = s
+    arrays["grad_sample"] = sample.cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, total
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    with open(os.path.join(path, "grad_names.txt"), "w") as f:
+        f.write("\n".join(nn_.param_names) + "\n")
+
+
+def measure_train(ctx, cfg_name, B, steps, warmup, headline=False, mixed_ratio=None, dump_dir=None):
+    """fwd+bwd sample-steps/s of one configuration at ctx.world GPUs; B = per-GPU batch. With `dump_dir`, what the
+    last timed step computed is written there (dump_outputs)."""
     from mdm_b200 import _lib, parallel
 
     pipe, nested = build_pipeline(cfg_name, ctx.dev, mixed_ratio)
@@ -209,21 +264,25 @@ def measure_train(ctx, cfg_name, B, steps, warmup, headline=False, mixed_ratio=N
                if ctx.world > 1 and os.environ.get("MDM_OVERLAP") is not None else None)
 
     def step(sample):
-        loss, *_ = pipe.get_loss(sample)
+        out = pipe.get_loss(sample)
         if overlap is not None:
             overlap.arm()
-        loss.mean().backward()
+        out[0].mean().backward()
         if overlap is not None:
             overlap.finish()
         elif ctx.world > 1:
             parallel.allreduce_gradients(vm)
-        return loss
+        return out
 
     def zero():
         vm.zero_grad(set_to_none=True)
 
+    last = []  # the outputs of the latest step, kept only for dump_dir
+
     def resident_step():
-        step(resident)
+        out = step(resident)
+        if dump_dir is not None:
+            last[:] = out
         zero()
 
     for _ in range(max(warmup, 3)):  # also sizes the engine's memory pool
@@ -233,12 +292,15 @@ def measure_train(ctx, cfg_name, B, steps, warmup, headline=False, mixed_ratio=N
     ms = timed(ctx, resident_step, steps)
     launches = _lib.launch_count() - l0
     clk = clocks.stop() if clocks is not None else None
+    if dump_dir is not None and ctx.rank == 0:
+        dump_outputs(dump_dir, last, vm)
+    del last[:]
     # ---- end to end: host (pinned) inputs, H2D inside the timed region, D2H of the loss
     loss_host = torch.empty(B).pin_memory()
 
     def e2e_step():
         sample = {k: v.to(ctx.dev, non_blocking=True) for k, v in host.items()}
-        loss = step(sample)
+        loss = step(sample)[0]
         loss_host.copy_(loss.detach(), non_blocking=True)
         zero()
 
@@ -401,10 +463,12 @@ def run_ours(args):
     if args.config != "cc12m_64x64" or args.batch:  # development: one named training config as the headline
         head, extra = measure_train(ctx, args.config, args.batch or {"cc12m_64x64": 64, "cc12m_256x256": 32,
                                                                        "cc12m_1024x1024": max(1, 8 // world)}[args.config],
-                                    args.steps, args.warmup, headline=True, mixed_ratio=args.mixed_ratio)
+                                    args.steps, args.warmup, headline=True, mixed_ratio=args.mixed_ratio,
+                                    dump_dir=args.dump_outputs)
         only = "headline"
     else:
-        head, extra = measure_train(ctx, "cc12m_64x64", 64, args.steps, args.warmup, headline=True)
+        head, extra = measure_train(ctx, "cc12m_64x64", 64, args.steps, args.warmup, headline=True,
+                                    dump_dir=args.dump_outputs)
     if only in (None, "cc12m_256x256_train"):
         configs["cc12m_256x256_train"], _ = measure_train(ctx, "cc12m_256x256", 32, max(3, args.steps // 4), 3)
         configs["cc12m_256x256_train"]["baseline_config"] = "BASELINE.json configs[2] (batch 32 per GPU, weak scaling)"
@@ -598,6 +662,8 @@ def main():
     ap.add_argument("--mixed-ratio", default=None, help="NestedDiffusionConfig.mixed_ratio for --config runs, e.g. 2:1")
     ap.add_argument("--only", default=None, help="headline | one key of the configs object (development aid)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the headline's last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

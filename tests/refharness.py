@@ -1,10 +1,11 @@
-"""Import the UNMODIFIED reference (apple/ml-mdm at /root/reference) on CPU so tests can pin the
-oracle against it and golden fixtures can be generated from it.
+"""Import the UNMODIFIED reference (apple/ml-mdm) on CPU so that the golden fixtures under tests/golden/ can be
+generated from it. The environment variable ML_MDM_ROOT names the directory of the checkout that holds the ml_mdm/
+package and configs/models/ (the ml-mdm-matryoshka tree). The tests themselves never import the reference: they
+compare against those fixtures.
 
-The reference's hot path needs five packages that carry no arithmetic and are not installed here
+The reference's hot path needs five packages that carry no arithmetic and may not be installed
 (torchinfo, simple_parsing, dataclass_wizard, mlx/mlx.data, boto3); they are stubbed in sys.modules
-before the import (SURVEY.md section 8c).  /root/reference does not exist on the GPU box: everything
-that uses this module must skip when `available()` is False.
+before the import (SURVEY.md section 8c).
 """
 import dataclasses
 import enum
@@ -13,7 +14,7 @@ import sys
 import types
 import typing
 
-REF_ROOT = "/root/reference/ml-mdm-matryoshka"
+REF_ROOT = os.environ.get("ML_MDM_ROOT", "")
 CFG_DIR = os.path.join(REF_ROOT, "configs", "models")
 
 
@@ -37,7 +38,7 @@ def load():
     if _loaded is not None:
         return _loaded
     if not available():
-        raise RuntimeError("reference tree not present")
+        raise RuntimeError("reference tree not present: set ML_MDM_ROOT to an apple/ml-mdm checkout")
     if "torchinfo" not in sys.modules:
         _mod("torchinfo", summary=lambda *a, **k: None)
     if "simple_parsing" not in sys.modules:

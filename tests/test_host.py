@@ -126,30 +126,63 @@ def test_plugin_overwrites_reference_registries():
     assert fake.MODEL_CONFIG_REGISTRY["nested2_unet_b200"]["model"] == "nested_unet_b200"
 
 
+def reference_config_module():
+    """A stand-in for the reference's ml_mdm.config, rebuilt from tests/golden/reference_configs.json: its model and
+    pipeline registries, get_model/get_pipeline (config.py:54-63), its config dataclasses and sampler enums (foreign
+    classes, not ours), and its config objects for cc12m_256x256 as the reference's own loader builds them from the
+    YAML (including its __post_init__ conversions)."""
+    import dataclasses
+    import enum
+    import json
+    import types
+    import typing
+
+    d = json.load(open(os.path.join(GOLD, "reference_configs.json")))
+    enums = {n: enum.Enum(n, members) for n, members in d["enums"].items()}
+    classes = {n: dataclasses.make_dataclass(n, [(f, typing.Any) for f in fields]) for n, fields in d["classes"].items()}
+
+    def dec(v):
+        if isinstance(v, dict) and "enum" in v:
+            return enums[v["enum"]][v["member"]]
+        if isinstance(v, dict) and "dataclass" in v:
+            return classes[v["dataclass"]](**{k: dec(x) for k, x in v["fields"].items()})
+        if isinstance(v, list):
+            return [dec(x) for x in v]
+        return v
+
+    m = types.SimpleNamespace(
+        MODEL_REGISTRY={k: object for k in d["MODEL_REGISTRY"]}, PIPELINE_REGISTRY={k: object for k in d["PIPELINE_REGISTRY"]},
+        MODEL_CONFIG_REGISTRY={k: {"model": v["model"], "config": classes[v["config"]]}
+                               for k, v in d["MODEL_CONFIG_REGISTRY"].items()},
+        PIPELINE_CONFIG_REGISTRY={k: classes[v] for k, v in d["PIPELINE_CONFIG_REGISTRY"].items()})
+    m.get_model = lambda name: m.MODEL_REGISTRY[m.MODEL_CONFIG_REGISTRY[name]["model"]]
+    m.get_pipeline = lambda name: m.PIPELINE_REGISTRY[m.MODEL_CONFIG_REGISTRY[name]["model"]]
+    return m, {k: dec(v) for k, v in d["cc12m_256x256"].items()}, classes, enums
+
+
 def test_plugin_on_live_reference_registry():
-    import refharness as rh
-
-    if not rh.available():
-        pytest.skip("reference tree not mounted")
-    ref = rh.load()
+    """Registration into the reference's registries, and the reference's own config objects (its dataclasses, its
+    ScheduleType/PredictionType/ThresholdType members) driving our NestedUNet and NestedDiffusion unchanged."""
     from mdm_b200 import plugin
+    from mdm_b200.diffusion import NestedDiffusion
 
-    saved = (dict(ref.config.MODEL_REGISTRY), dict(ref.config.PIPELINE_REGISTRY))
-    try:
-        plugin.register(ref.config)
-        assert ref.config.get_model("nested2_unet") is NestedUNet
-        assert ref.config.get_model("unet") is UNet
-        # the reference's own config dataclass drives our constructor unchanged
-        y = rh.load_yaml("cc12m_256x256.yaml")
-        ucfg = rh.from_dict(ref.config.MODEL_CONFIG_REGISTRY["nested_unet"]["config"], y["unet_config"])
-        ucfg.conditioning_feature_dim = 2048
-        ucfg.initialize_inner_with_pretrained = None
-        with torch.device("meta"):
-            m = ref.config.get_model("nested_unet")(3, 3, ucfg)
-        assert m.nest_ratio == [4] and len(m.state_dict()) == 889
-        dcfg = rh.from_dict(ref.config.PIPELINE_CONFIG_REGISTRY["nested_unet"], y["diffusion_config"])
-        pipe = ref.config.get_pipeline("nested_unet")(m, dcfg)
-        assert pipe.sampler.gammas.shape == (1001,)
-    finally:
-        ref.config.MODEL_REGISTRY.clear(); ref.config.MODEL_REGISTRY.update(saved[0])
-        ref.config.PIPELINE_REGISTRY.clear(); ref.config.PIPELINE_REGISTRY.update(saved[1])
+    ref, cfgs, classes, enums = reference_config_module()
+    plugin.register(ref)
+    assert ref.get_model("nested2_unet") is NestedUNet
+    assert ref.get_model("unet") is UNet
+    assert ref.get_pipeline("nested_unet") is NestedDiffusion
+    ucfg = cfgs["unet_config"]
+    assert type(ucfg) is ref.MODEL_CONFIG_REGISTRY["nested_unet"]["config"] is classes["NestedUNetConfig"]
+    ucfg.conditioning_feature_dim = 2048
+    ucfg.initialize_inner_with_pretrained = None
+    with torch.device("meta"):
+        m = ref.get_model("nested_unet")(3, 3, ucfg)
+    assert m.nest_ratio == [4] and len(m.state_dict()) == 889
+    dcfg = cfgs["diffusion_config"]
+    assert type(dcfg) is ref.PIPELINE_CONFIG_REGISTRY["nested_unet"]
+    assert type(dcfg.sampler_config.schedule_type) is enums["ScheduleType"]  # a foreign enum member
+    pipe = ref.get_pipeline("nested_unet")(m, dcfg)
+    assert pipe.sampler.gammas.shape == (1001,)
+    tab = pipe.sampler.gammas
+    want = samplers.Sampler(mc.SamplerConfig(num_diffusion_steps=1000, schedule_type="DEEPFLOYD")).gammas
+    assert torch.equal(tab, want)  # DEEPFLOYD, taken from the foreign enum member by name

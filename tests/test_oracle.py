@@ -1,6 +1,8 @@
 """Pins the oracle (oracle/*.py) against the golden fixtures generated from the unmodified reference
-(tests/golden/make_golden.py) and, when /root/reference is present, against the reference live."""
+(tests/golden/make_golden.py)."""
 import copy
+import hashlib
+import json
 import os
 import types
 
@@ -8,7 +10,6 @@ import numpy as np
 import pytest
 import torch
 
-import refharness as rh
 import tiny_configs as tc
 from oracle import diffusion_ref as dref
 from oracle import unet_ref
@@ -151,138 +152,141 @@ def test_schedule_tables_and_timesteps_bit_exact():
     assert len(ts) == 51 and list(ts[:4]) == [981, 962, 942, 922] and list(ts[-4:]) == [59, 39, 20, 0]
 
 
-@pytest.mark.skipif(not rh.available(), reason="reference tree not mounted (GPU box)")
+# (tokens, seed) of the full-width cases; batch 1, parameters and inputs from numpy seeds
+SHIPPED = {"cc12m_64x64": (16, 0), "cc12m_256x256": (8, 1), "cc12m_1024x1024": (4, 2)}
+SHIPPED_SAMPLE = 2048
+
+
+def shipped_case(name):
+    """Parameters (every tensor of the state_dict seeded, tc.seeded_state_dict) and inputs of one shipped config at
+    full width; shapes come from the product's module tree, which test_host pins to the reference's state_dict."""
+    import yaml
+
+    from mdm_b200 import config as mc
+    from mdm_b200.models import NestedUNet, UNet
+
+    path = os.path.join(os.path.dirname(GOLD), "..", "ml-mdm_b200", "mdm_b200", "configs", name + ".yaml")
+    ucfg, _, nested = mc.load_yaml_configs(path)
+    with torch.device("meta"):
+        m = (NestedUNet if nested else UNet)(3, 3, ucfg)
+    tokens, seed = SHIPPED[name]
+    P = tc.seeded_state_dict(m.state_dict(), seed)
+    res = int(name.split("_")[1].split("x")[0])
+    nlev = {64: 1, 256: 2, 1024: 3}[res]
+    x, t, lm, mask = tc.seeded_inputs(seed, 1, res, tokens, lm_dim=2048, nlevels=nlev)
+    return yaml.safe_load(open(path)), P, x, t, lm, mask, nested
+
+
+def strip_pretrained(d):
+    """Nested config dicts: no pretrained initialisation anywhere."""
+    if isinstance(d, dict):
+        if "initialize_inner_with_pretrained" in d:
+            d["initialize_inner_with_pretrained"] = None
+        for v in d.values():
+            strip_pretrained(v)
+    return d
+
+
+def check_shipped(name):
+    """Oracle forward vs the reference modules' forward on the same parameters and inputs. The reference's outputs
+    are stored at fixed sample positions and as means over each image row."""
+    y, P, x, t, lm, mask, nested = shipped_case(name)
+    gold = np.load(os.path.join(GOLD, f"shipped_{name}.npz"))
+    net = unet_ref.OracleNet(ns(strip_pretrained(copy.deepcopy(y["unet_config"]))), 2048)
+    with torch.no_grad():
+        out = net.forward(P, x, t, lm, mask, {})
+    out = list(out) if nested else [out]
+    assert len(out) == len([k for k in gold.files if k.startswith("sample")])
+    for i, o in enumerate(out):
+        assert list(o.shape) == list(gold[f"shape{i}"])
+        close(tc.golden_sample(o, SHIPPED_SAMPLE, seed=i), gold[f"sample{i}"], 1e-5)
+        close(o.mean(dim=3), gold[f"rowmean{i}"], 1e-5)
+
+
 def test_oracle_matches_live_reference_on_shipped_64_config():
     """cc12m_64x64 at full width (461 M parameters), B=1, S=16: oracle vs the reference modules."""
-    torch.manual_seed(0)
-    y = rh.load_yaml("cc12m_64x64.yaml")
-    model, _ = rh.build(y["unet_config"], y["diffusion_config"], "unet", 2048)
-    with torch.no_grad():
-        for p in model.parameters():
-            if float(p.abs().max()) == 0:
-                p.normal_(0, 0.02)  # zero-initialised layers would hide most of the network
-    ucfg = copy.deepcopy(y["unet_config"])
-    net = unet_ref.OracleNet(ns(ucfg), 2048)
-    x = torch.randn(1, 3, 64, 64)
-    t = torch.tensor([417])
-    lm = torch.randn(1, 16, 2048)
-    mask = torch.ones(1, 16)
-    with torch.no_grad():
-        ref = model(x, t, lm, mask, {})
-        out = net.forward(dict(model.state_dict()), x, t, lm, mask, {})
-    close(out, ref, 1e-5)
+    check_shipped("cc12m_64x64")
 
 
-@pytest.mark.skipif(not rh.available(), reason="reference tree not mounted (GPU box)")
 def test_oracle_matches_live_reference_on_shipped_256_config():
     """cc12m_256x256 at full width (2-level nest, 476.6 M parameters), B=1, S=8: oracle vs the reference's
     NestedUNet — pins the nesting adapters, the inner/outer skip wiring and the 4x resolution ratio at the real
     channel widths (the tiny nested fixture pins them at toy widths)."""
-    torch.manual_seed(1)
-    y = rh.load_yaml("cc12m_256x256.yaml")
-    model, _ = rh.build(y["unet_config"], y["diffusion_config"], "nested_unet", 2048)
-    with torch.no_grad():
-        for p in model.parameters():
-            if float(p.abs().max()) == 0:
-                p.normal_(0, 0.02)
-    ucfg = copy.deepcopy(y["unet_config"])
-    ucfg["initialize_inner_with_pretrained"] = None
-    net = unet_ref.OracleNet(ns(ucfg), 2048)
-    xs = [torch.randn(1, 3, 256, 256), torch.randn(1, 3, 64, 64)]
-    t = torch.tensor([233])
-    lm = torch.randn(1, 8, 2048)
-    mask = torch.ones(1, 8)
-    with torch.no_grad():
-        ref = model(xs, t, lm, mask, {})
-        out = net.forward(dict(model.state_dict()), xs, t, lm, mask, {})
-    assert len(out) == len(ref) == 2
-    for o, r in zip(out, ref):
-        assert o.shape == r.shape
-        close(o, r, 1e-5)
+    check_shipped("cc12m_256x256")
 
 
-@pytest.mark.skipif(not rh.available(), reason="reference tree not mounted (GPU box)")
 def test_oracle_matches_live_reference_on_shipped_1024_config():
     """cc12m_1024x1024 at full width (3-level nest, 481 M parameters), B=1, S=4: oracle vs the reference."""
-    torch.manual_seed(2)
-    y = rh.load_yaml("cc12m_1024x1024.yaml")
-    model, _ = rh.build(y["unet_config"], y["diffusion_config"], "nested2_unet", 2048)
-    with torch.no_grad():
-        for p in model.parameters():
-            if float(p.abs().max()) == 0:
-                p.normal_(0, 0.02)
-
-    def strip(d):  # nested dicts: no pretrained initialisation anywhere
-        if isinstance(d, dict):
-            if "initialize_inner_with_pretrained" in d:
-                d["initialize_inner_with_pretrained"] = None
-            for v in d.values():
-                strip(v)
-        return d
-
-    net = unet_ref.OracleNet(ns(strip(copy.deepcopy(y["unet_config"]))), 2048)
-    xs = [torch.randn(1, 3, 1024, 1024), torch.randn(1, 3, 256, 256), torch.randn(1, 3, 64, 64)]
-    t = torch.tensor([77])
-    lm = torch.randn(1, 4, 2048)
-    mask = torch.ones(1, 4)
-    with torch.no_grad():
-        ref = model(xs, t, lm, mask, {})
-        out = net.forward(dict(model.state_dict()), xs, t, lm, mask, {})
-    assert len(out) == len(ref) == 3
-    for o, r in zip(out, ref):
-        assert o.shape == r.shape
-        close(o, r, 1e-5)
+    check_shipped("cc12m_1024x1024")
 
 
-@pytest.mark.skipif(not rh.available(), reason="reference tree not mounted (GPU box)")
+MIXED_B = 3
+GRAD_SAMPLE = 64  # gradient elements stored per parameter: the whole gradient for 242 of the 461
+
+
 def test_oracle_mixed_ratio_loss_matches_live_reference():
     """NestedDiffusion.get_loss with mixed_ratio='2:1' (what configs/models/cc12m_256x256.yaml:108 sets): only the
     leading int(2/3 * B) samples run the high-resolution level, predictions are zero-padded, the per-level loss is
     divided by the fraction and masked (diffusion.py:262-274, 378-382; nested_unet.py:180,193-204,209). The oracle
-    replays the reference's CPU generator draws; loss and every gradient are compared."""
-    B = 3
-    dcfg = copy.deepcopy(tc.TINY_NESTED_DIFFUSION)
-    dcfg["mixed_ratio"] = "2:1"
-    ucfg = copy.deepcopy(tc.TINY_NESTED)
-    model, pipe = rh.build(ucfg, dcfg, "nested_unet", tc.LM_DIM)
-    sd = tc.seeded_state_dict(model.state_dict(), 7)
-    model.load_state_dict(sd)
+    replays the reference's CPU generator draws; loss, x_t and every gradient (its norm, and GRAD_SAMPLE elements
+    at fixed positions) are compared with what the reference computed."""
+    B = MIXED_B
+    gold = np.load(os.path.join(GOLD, "tiny_nested_mixed.npz"))
+    names = open(os.path.join(GOLD, "tiny_nested_params.txt")).read().split()
+    P = params_for("nested", names, requires_grad=True)
     x, t, lm, mask = tc.seeded_inputs(3, B, 32, 6, nlevels=2)
     images = x[0].clamp(-1, 1)
-    torch.manual_seed(4321)
-    pipe.train()
-    loss, time, x_t, pred, tgt, _ = pipe.get_loss({"images": images, "lm_outputs": lm, "lm_mask": mask})
-    loss.mean().backward()
-    torch.manual_seed(4321)
-    time_r = torch.randint(0, 1000, (B,))
+    torch.manual_seed(4321)  # the draws of the reference's get_loss
+    time = torch.randint(0, 1000, (B,))
     eps = [torch.randn_like(images), None]
     eps[1] = torch.empty(B, 3, 8, 8).normal_()
-    assert torch.equal(time_r, time)
+    assert np.array_equal(time.numpy(), gold["time"])
     ocfg = copy.deepcopy(tc.TINY_NESTED)
     ocfg["initialize_inner_with_pretrained"] = None
     net = unet_ref.OracleNet(ns(ocfg), tc.LM_DIM)
-    P = {k: v.clone().requires_grad_(True) for k, v in sd.items()}
     gam = dref.gammas_f32("DEEPFLOYD", 1000)
     mr = dref.mixed_ratio_fractions("2:1")
     assert int(mr[0] * B) == 2 and mr[1] == 1.0
     oloss, ox_t, _ = dref.training_loss(net, P, images, eps, time, lm, mask, gam, [4, 1], dref.V_PREDICTION, dref.DDPM,
                                         shifted=True, power=1, mixed_ratio=mr)
-    close(ox_t[0], x_t, 1e-6)
-    close(oloss, loss.detach())
+    close(ox_t[0], gold["x_t"], 1e-6)
+    close(oloss.detach(), gold["loss"])
     oloss.mean().backward()
-    for k, p in model.named_parameters():
-        close(P[k].grad, p.grad, 2e-4)
+    # Biases in front of a GroupNorm get gradients that are mathematically zero (the reference's are below 4e-8,
+    # every other one above 1e-3): their values are rounding noise, which differs between CPUs. Those must stay
+    # below 1e-3 of the median gradient norm; every other gradient is compared with the reference's.
+    norms = np.array([float(P[k].grad.norm()) for k in names])
+    ref = gold["grad_norms"]
+    zero = ref < 1e-3 * np.median(ref)
+    assert np.all(norms[zero] < 1e-3 * np.median(ref))
+    assert np.max(np.abs(norms - ref)[~zero] / ref[~zero]) < 1e-3
+    for i, k in enumerate(names):  # close() of the whole gradient, at the stored positions
+        if zero[i]:
+            continue
+        got = tc.golden_sample(P[k].grad, GRAD_SAMPLE, seed=i).double()
+        want = torch.from_numpy(gold["grad_sample"][i, :got.numel()]).double()
+        assert float((got - want).abs().max()) <= 2e-4 * float(gold["grad_absmax"][i]), k
 
 
-@pytest.mark.skipif(not rh.available(), reason="reference tree not mounted (GPU box)")
-@pytest.mark.parametrize("mode", ["DYNAMIC", "DYNAMIC_IF", "CLIP", "NONE"])
-def test_oracle_clip_sample_matches_live_reference(mode):
-    """Sampler.clip_sample incl. dynamic thresholding (samplers.py:461-508): bit-identical restatement."""
-    ref = rh.load()
-    cfg = ref.samplers.SamplerConfig()
-    smp = ref.samplers.Sampler(cfg)
-    cfg.threshold_function = getattr(ref.samplers.ThresholdType, mode)
+CLIP_MODES = ["DYNAMIC", "DYNAMIC_IF", "CLIP", "NONE"]
+
+
+def clip_input():
     g = torch.Generator().manual_seed(3)
-    x = torch.randn(3, 3, 32, 32, generator=g) * torch.tensor([0.4, 1.3, 9.0]).view(3, 1, 1, 1)
+    return torch.randn(3, 3, 32, 32, generator=g) * torch.tensor([0.4, 1.3, 9.0]).view(3, 1, 1, 1)
+
+
+def digest(t):
+    return hashlib.sha256(t.contiguous().numpy().tobytes()).hexdigest()
+
+
+@pytest.mark.parametrize("mode", CLIP_MODES)
+def test_oracle_clip_sample_matches_live_reference(mode):
+    """Sampler.clip_sample incl. dynamic thresholding (samplers.py:461-508): bit-identical restatement, checked
+    against the SHA-256 of the reference's float32 output bytes."""
+    want = json.load(open(os.path.join(GOLD, "clip_sample.json")))[mode]
+    x = clip_input()
     for scale in (1.0, 4.0):
-        assert torch.equal(smp.clip_sample(x, scale), dref.clip_sample(x, scale, mode if mode != "NONE" else False))
+        out = dref.clip_sample(x, scale, mode if mode != "NONE" else False)
+        assert out.dtype == torch.float32 and out.shape == x.shape
+        assert digest(out) == want[str(scale)], (mode, scale)

@@ -102,6 +102,16 @@ def seeded_state_dict(ref_state_dict, seed, std=0.05):
     return out
 
 
+def golden_sample(t, n, seed=0):
+    """`n` elements of a flattened tensor at fixed, seeded positions (all of it when it has no more than `n`):
+    outputs too large to commit whole are stored and compared at these positions."""
+    flat = torch.as_tensor(t).detach().reshape(-1)
+    if flat.numel() <= n:
+        return flat.clone()
+    idx = np.sort(np.random.default_rng(seed).choice(flat.numel(), n, replace=False))
+    return flat[torch.from_numpy(idx)]
+
+
 def seeded_inputs(seed, batch, res, tokens, lm_dim=LM_DIM, nlevels=1, ratio=4):
     rng = np.random.default_rng(seed)
     xs = []
